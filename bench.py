@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- frames/sec of the volumetric renderer hot path on B200 (BASELINE.json metric).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--precision fp16|fp32]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--precision fp16|fp32] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 A "step" is ONE 512x512 frame of the north-star synthetic workload (SURVEY.md section 8d "512x512x128"): head+torso model of the
@@ -19,6 +19,9 @@ roofline: dominant kernel = the field kernel (grid gathers + MLPs); achieved = s
          gather rate as the metric asks; tensor-pipe fraction is reported beside it.
 cpu_baseline: the CPU oracle (port of the reference path, OpenMP + numpy, all host threads) on a bounded sample of the SAME
          frame (rays x 128 samples), extrapolated to frames/s.
+--dump-outputs DIR: after the timed steps, what the last timed step returned to its caller (the RGB8 frame and the frame counters)
+         is written as DIR/<name>.npy in float32 / float64.  The inputs depend only on the arguments, so two builds can be compared
+         output for output.
 --impl reference: the reference's CPU implementation timed on the host cores (rank 0 only): the oracle port of the RAD-NeRF
          path on a bounded sample per step; the vanilla AD-NeRF (modules/nerfs) port is reported in `adnerf_cpu`.
 """
@@ -176,7 +179,7 @@ def run_reference_arm(args, rank):
     """--impl reference: the reference path on the host CPU (rank 0 only)."""
     if rank != 0:
         return
-    steps, warm = max(1, args.steps), args.warmup
+    steps, warm = args.steps, args.warmup
     t0 = time.perf_counter()
     for _ in range(max(1, warm)):
         _cpu_port_once(256, host_threads())                         # warm-up steps: library load, page faults, thread pools
@@ -186,8 +189,6 @@ def run_reference_arm(args, rank):
     for _ in range(steps):
         fps, dt, threads, sample = cpu_port_fps(CPU_SAMPLE_RAYS, warm=False)
         fps_list.append(fps)
-        if time.perf_counter() - t0 > 150:
-            break
     k = len(fps_list)
     value = k / sum(1.0 / f for f in fps_list)
     line = {"impl": "reference", "metric": METRIC, "value": value, "unit": "frames/s", "n_gpus": args.gpus, "steps": k, "warmup": 1,
@@ -269,6 +270,16 @@ def gather_probe_gbs(model, fi, dev, precision):
             "what": "gf_gather_probe: the producers' gather code alone (no MLP, full occupancy) over one 8.4 M-sample round of this frame"}
 
 
+def dump_outputs(directory, arrays):
+    """Write each array as DIR/<name>.npy: integer and float64 data as float64, everything else as float32."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        a = a.astype(np.float64 if a.dtype in (np.int64, np.uint64, np.float64) else np.float32)
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -282,7 +293,12 @@ def main():
     ap.add_argument("--no-ref-cuda", action="store_true")
     ap.add_argument("--no-may", action="store_true", help="skip the May-configuration / AD-NeRF context measurements")
     ap.add_argument("--eager", action="store_true", help="per-frame eager launches instead of CUDA-graph replay (A/B)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy (frame configurations only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config in ("seq300", "train")):
+        ap.error("--dump-outputs applies to the GPU frame configurations (%s)" % ", ".join(sorted(CONFIGS)))
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -380,6 +396,8 @@ def main():
     ev1.record()
     barrier()
     ms_res = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"rgb8": rgb8.view(H, W, 3), "counters": counters})
     # ---- timed: end to end (host inputs, host result), 3 repeats of the K-frame sequence, median ----
     e2e_ms = []
     for rep in range(3):

@@ -92,13 +92,14 @@ def build_one(name, verbose=False):
     shutil.copy(os.path.join(bdir, name + ".so"), os.path.join(OUT, name + ".so"))
 
 
-def main():
+def main(names=()):
+    """Build the named extensions (all four by default); a no-op where the reference tree is absent."""
     if not os.path.isdir(REF):
         print("reference tree not present (%s): skipping oracle/_ref build" % REF)
         return 0
     os.makedirs(OUT, exist_ok=True)
     mirror_python()
-    names = sys.argv[1:] or list(EXTS)
+    names = list(names) or list(EXTS)
     for n in names:
         if built(n):
             print("[oracle/_ref] %s already built" % n)
@@ -110,4 +111,4 @@ def main():
 
 
 if __name__ == "__main__":
-    sys.exit(main())
+    sys.exit(main(sys.argv[1:]))

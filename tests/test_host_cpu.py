@@ -6,6 +6,8 @@ import numpy as np
 import pytest
 import torch
 
+import refgold
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -40,19 +42,23 @@ def test_rays_poses_bgcoords_match_oracle_restatement():
             utils.get_rays(fi['pose'], fi['intrinsics'], 33, 47)
     # the three pixel-sampling modes select exactly the pixels the reference's get_rays selects under the same torch seed
     from oracle import ref_model
-    if ref_model.available():
-        ns = ref_model.load()
-        for kw in (dict(N=40), dict(N=64, patch_size=4), dict(rect=(2, 7, 3, 9)), dict(N=10 ** 6)):
+    R = refgold.Reference("pixel_indices_audio_features", ref_model.available())
+    ns = ref_model.load() if R.live else None
+    for n, kw in enumerate((dict(N=40), dict(N=64, patch_size=4), dict(rect=(2, 7, 3, 9)), dict(N=10 ** 6))):
+        if R.live:
             torch.manual_seed(3)
-            ref = ns.utils.get_rays(torch.eye(4)[None], (20., 20., 8., 8.), 16, 24, **kw)['inds'][0]
-            torch.manual_seed(3)
-            ours = utils.pixel_indices(16, 24, kw.get('N', -1), kw.get('patch_size', 1), kw.get('rect'))
-            assert torch.equal(ref, ours), kw
-        f = torch.randn(9, 1, 204)
+            R.put(f"inds_{n}", ns.utils.get_rays(torch.eye(4)[None], (20., 20., 8., 8.), 16, 24, **kw)['inds'][0])
+        torch.manual_seed(3)
+        ours = utils.pixel_indices(16, 24, kw.get('N', -1), kw.get('patch_size', 1), kw.get('rect'))
+        assert np.array_equal(R[f"inds_{n}"], ours.numpy()) and R[f"inds_{n}"].dtype == ours.numpy().dtype, kw
+    f = torch.randn(9, 1, 204, generator=torch.Generator().manual_seed(4))
+    if R.live:
         ns.hparams['smo_win_size'] = 5
-        for mode in (0, 1, 2):
-            for idx in range(9):
-                assert torch.equal(utils.get_audio_features(f, mode, idx, 5), ns.utils.get_audio_features(f, mode, idx)), (mode, idx)
+    for mode in (0, 1, 2):
+        for idx in range(9):
+            if R.live:
+                R.put(f"audio_{mode}_{idx}", ns.utils.get_audio_features(f, mode, idx), rows="digest")
+            assert R.equal(f"audio_{mode}_{idx}", utils.get_audio_features(f, mode, idx, 5)), (mode, idx)
     assert np.allclose(utils.convert_poses(fi['pose'])[0].numpy(), OF.convert_poses(fi['pose'][0].numpy()), atol=1e-6)
     assert np.allclose(utils.get_bg_coords(33, 47, 'cpu')[0].numpy(), OF.get_bg_coords(33, 47), atol=1e-7)
     p0 = utils.orbit_pose(3.35, 0.0)

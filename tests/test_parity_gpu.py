@@ -1,6 +1,7 @@
 """GPU parity tests: every libgfrender op and the fused frame renderer, through the C ABI (via the Python mirror),
 against (a) the CPU oracle (oracle/gf_oracle.c + oracle/field.py) and (b) when oracle/_ref/*.so is present, the
-UNMODIFIED reference kernels running on the same GPU.
+UNMODIFIED reference kernels running on the same GPU, or, where they are not built, their outputs recorded under
+tests/golden/reference/ (tests/refgold.py).
 
 Bars (north_star): integer outputs (occupancy indices, per-ray sample counts, termination slots, alive flags)
 bit-exact; floating outputs within 1e-3 relative per pixel (abs floor 1e-5); where our fp32 arithmetic mirrors
@@ -10,6 +11,7 @@ import numpy as np
 import pytest
 import torch
 
+import refgold
 import scenes
 from conftest import ref_ext
 
@@ -70,12 +72,14 @@ def test_near_far_and_march_bit_exact(rm, oracle_ops, bound, C):
     nears, fars = rm.near_far_from_aabb(cu(o), cu(d), cu(aabb), 0.05)
     assert bits_equal(nears.cpu().numpy(), n_ref) and bits_equal(fars.cpu().numpy(), f_ref)
     RM = ref_ext("_raymarching_face")
-    if RM is not None:
+    R = refgold.Reference(f"march_b{bound:g}_c{C}", RM is not None)
+    if R.live:
         n2 = torch.empty(N, device="cuda"); f2 = torch.empty(N, device="cuda")
         RM.near_far_from_aabb(cu(o), cu(d), cu(aabb), N, 0.05, n2, f2)
-        assert torch.equal(n2, nears) and torch.equal(f2, fars)
-    for bf in (scenes.random_bitfield(C, H, 0.3, 1), scenes.full_bitfield(C, H), scenes.random_bitfield(C, H, 0.03, 2)):
-        for n_step, dt_gamma, max_steps, noisy in ((4, 1 / 256, 16, False), (8, 0.0, 128, False), (3, 1 / 128, 1024, True)):
+        R.put("nears", n2, rows="digest"); R.put("fars", f2, rows="digest")
+    assert R.equal("nears", nears) and R.equal("fars", fars)
+    for ib, bf in enumerate((scenes.random_bitfield(C, H, 0.3, 1), scenes.full_bitfield(C, H), scenes.random_bitfield(C, H, 0.03, 2))):
+        for ic, (n_step, dt_gamma, max_steps, noisy) in enumerate(((4, 1 / 256, 16, False), (8, 0.0, 128, False), (3, 1 / 128, 1024, True))):
             noises = np.random.RandomState(5).rand(N).astype(np.float32) if noisy else np.zeros(N, np.float32)
             alive = np.arange(N, dtype=np.int32)
             x_ref, _, dl_ref, idx_ref = oracle_ops.march_rays(N, n_step, alive, n_ref, o, d, bound, bf, C, H, n_ref, f_ref, 128, noises, dt_gamma,
@@ -89,10 +93,12 @@ def test_near_far_and_march_bit_exact(rm, oracle_ops, bound, C):
                                                 _lib.stream_ptr()))
             assert bits_equal(xyzs.cpu().numpy(), x_ref), "march xyzs differ from oracle"
             assert bits_equal(deltas.cpu().numpy(), dl_ref), "march deltas differ from oracle"
-            if RM is not None:
+            if R.live:
                 x2 = torch.zeros(M, 3, device="cuda"); d2_ = torch.zeros(M, 3, device="cuda"); l2 = torch.zeros(M, 2, device="cuda")
                 RM.march_rays(N, n_step, cu(alive), nears, cu(o), cu(d), bound, dt_gamma, max_steps, C, H, cu(bf), nears, fars, x2, d2_, l2, cu(noises))
-                assert torch.equal(x2, xyzs) and torch.equal(l2, deltas) and torch.equal(d2_, dirs), "march differs from compiled reference"
+                for k, v in (("xyzs", x2), ("deltas", l2), ("dirs", d2_)):
+                    R.put(f"{k}_{ib}_{ic}", v, rows="digest")
+            assert all(R.equal(f"{k}_{ib}_{ic}", v) for k, v in (("xyzs", xyzs), ("deltas", deltas), ("dirs", dirs))), "march differs from compiled reference"
 
 
 def test_composite_rays_vs_oracle_and_reference(rm, oracle_ops):
@@ -119,11 +125,14 @@ def test_composite_rays_vs_oracle_and_reference(rm, oracle_ops):
     assert np.array_equal(a.cpu().numpy()[~edge], a_ref[~edge])
     assert_close(ws.cpu().numpy(), ws_ref, what="ws"); assert_close(dep.cpu().numpy(), dep_ref, what="depth"); assert_close(img.cpu().numpy(), img_ref, what="img")
     RM = ref_ext("_raymarching_face")
-    if RM is not None:
+    R = refgold.Reference("composite_rays", RM is not None)
+    if R.live:
         a2, t2, ws2, dep2, img2 = cu(alive), cu(t0), cu(ws0), cu(dep0), cu(img0)
         RM.composite_rays(N, n_step, 1e-4, a2, t2, cu(sig), cu(rgb), cu(deltas), ws2, dep2, img2)
-        assert torch.equal(a2, a) and torch.equal(t2, t), "termination flags / rays_t differ from compiled reference"
-        assert torch.equal(ws2, ws) and torch.equal(dep2, dep) and torch.equal(img2, img), "composite floats differ from compiled reference"
+        for k, v in (("alive", a2), ("t", t2), ("ws", ws2), ("depth", dep2), ("image", img2)):
+            R.put(k, v, rows="digest")
+    assert R.equal("alive", a) and R.equal("t", t), "termination flags / rays_t differ from compiled reference"
+    assert R.equal("ws", ws) and R.equal("depth", dep) and R.equal("image", img), "composite floats differ from compiled reference"
 
 
 def test_march_rays_train_and_composite_train(rm, oracle_ops):
@@ -132,7 +141,9 @@ def test_march_rays_train_and_composite_train(rm, oracle_ops):
     aabb = scenes.aabb_of(bound)
     bf = scenes.random_bitfield(C, H, 0.3, 1)
     nears_np, fars_np = oracle_ops.near_far_from_aabb(o, d, aabb, 0.05)
-    for max_steps, dt_gamma in ((16, 1 / 256), (64, 0.0)):
+    RM = ref_ext("_raymarching_face")
+    R = refgold.Reference("march_rays_train", RM is not None)
+    for it, (max_steps, dt_gamma) in enumerate(((16, 1 / 256), (64, 0.0))):
         noises = np.random.RandomState(6).rand(N).astype(np.float32)
         noises[0] = 0.0            # allocation order is rotated by bits(noises[0]) (checked separately below): 0 = plain index order
         x_ref, d_ref, dl_ref, rays_ref, cnt_ref = oracle_ops.march_rays_train(o, d, bound, bf, C, H, nears_np, fars_np, noises, dt_gamma, max_steps)
@@ -146,18 +157,18 @@ def test_march_rays_train_and_composite_train(rm, oracle_ops):
         # deterministic layout == the oracle's ray-order layout: direct equality
         assert np.array_equal(rays.cpu().numpy(), rays_ref) and np.array_equal(counter.cpu().numpy(), cnt_ref)
         assert bits_equal(xyzs.cpu().numpy(), x_ref) and bits_equal(deltas.cpu().numpy(), dl_ref) and bits_equal(dirs.cpu().numpy(), d_ref)
-        RM = ref_ext("_raymarching_face")
-        if RM is not None:   # reference layout is atomics-ordered: compare per ray
+        if R.live:   # reference layout is atomics-ordered: compare per ray
             x2 = torch.zeros(M, 3, device="cuda"); dd2 = torch.zeros(M, 3, device="cuda"); l2 = torch.zeros(M, 2, device="cuda")
             r2 = torch.empty(N, 3, dtype=torch.int32, device="cuda"); c2 = torch.zeros(2, dtype=torch.int32, device="cuda")
             RM.march_rays_train(cu(o), cu(d), cu(bf), bound, dt_gamma, max_steps, N, C, H, M, cu(nears_np), cu(fars_np), x2, dd2, l2, r2, c2, cu(noises))
             r2n = r2.cpu().numpy(); r2n = r2n[np.argsort(r2n[:, 0])]
-            assert np.array_equal(r2n[:, 2], rays_ref[:, 2]) and np.array_equal(c2.cpu().numpy(), cnt_ref)
+            R.put(f"counts_{it}", r2n[:, 2]); R.put(f"counter_{it}", c2)
             x2n, l2n = x2.cpu().numpy(), l2.cpu().numpy()
-            for i in range(0, N, 37):
-                c = rays_ref[i, 2]
-                assert bits_equal(x2n[r2n[i, 1]:r2n[i, 1] + c], x_ref[rays_ref[i, 1]:rays_ref[i, 1] + c])
-                assert bits_equal(l2n[r2n[i, 1]:r2n[i, 1] + c], dl_ref[rays_ref[i, 1]:rays_ref[i, 1] + c])
+            R.put(f"xyzs_{it}", np.concatenate([x2n[r2n[i, 1]:r2n[i, 1] + r2n[i, 2]] for i in range(0, N, 37)]), rows="digest")
+            R.put(f"deltas_{it}", np.concatenate([l2n[r2n[i, 1]:r2n[i, 1] + r2n[i, 2]] for i in range(0, N, 37)]), rows="digest")
+        assert np.array_equal(R[f"counts_{it}"], rays_ref[:, 2]) and np.array_equal(R[f"counter_{it}"], cnt_ref)
+        for k, v in ((f"xyzs_{it}", x_ref), (f"deltas_{it}", dl_ref)):
+            assert R.equal(k, np.concatenate([v[rays_ref[i, 1]:rays_ref[i, 1] + rays_ref[i, 2]] for i in range(0, N, 37)])), k
         # rotated allocation order (overflow then drops a pseudo-random run of rays, not always the highest indices): same per-ray
         # samples, offsets = exclusive scan of the counts starting at ray rot = (bits(noises[0]) >> 3) % N; with M too small the
         # dropped rays are exactly those whose offset + count exceeds M (raymarching.cu:457)
@@ -198,11 +209,15 @@ def test_march_rays_train_and_composite_train(rm, oracle_ops):
         assert_close(r_t.grad.cpu().numpy()[:Mtot], gr_r[:Mtot], what="grad_rgbs")
         assert_close(a_t.grad.cpu().numpy()[:Mtot], ga_r[:Mtot], what="grad_ambient")
         assert_close(s_t.grad.cpu().numpy()[:Mtot], gs_r[:Mtot], rel=2e-3, abs_=1e-4 * np.abs(gs_r).max(), what="grad_sigmas")
-        if RM is not None:
+        if R.live:
             g1 = torch.zeros(M, device="cuda"); g2 = torch.zeros(M, 3, device="cuda"); g3 = torch.zeros(M, device="cuda")
             RM.composite_rays_train_backward(cu(gws), cu(gamb), cu(gimg), cu(sig), cu(rgb), cu(amb), deltas, rays, w2.detach(), a2.detach(), i2.detach(), M, N, 1e-4, g1, g2, g3)
-            assert_close(s_t.grad.cpu().numpy(), g1.cpu().numpy(), rel=1e-4, abs_=1e-5 * float(g1.abs().max()), what="grad_sigmas vs reference")
-            assert torch.equal(g2, r_t.grad)
+            R.put(f"grad_sigmas_{it}", g1, rows=np.random.RandomState(it).choice(Mtot, min(Mtot, 1024), replace=False))
+            R.put(f"grad_sigmas_max_{it}", g1.abs().max())
+            R.put(f"grad_rgbs_{it}", g2, rows="digest")
+        assert_close(s_t.grad.cpu().numpy()[R.rows(f"grad_sigmas_{it}")], R[f"grad_sigmas_{it}"], rel=1e-4,
+                     abs_=1e-5 * float(R[f"grad_sigmas_max_{it}"]), what="grad_sigmas vs reference")
+        assert R.equal(f"grad_rgbs_{it}", r_t.grad)
 
 
 def test_utils_ops(rm, oracle_ops):
@@ -239,14 +254,16 @@ def test_grid_encoder(oracle_ops, D, gridtype, interp):
     bad = np.abs(dyn - dy_ref) > 1e-3 * float(np.abs(dy_ref).max()) + 2e-3 * np.abs(dy_ref)
     assert bad.mean() < 2e-3, f"grid dy_dx vs oracle: {bad.sum()} of {bad.size} entries differ"
     GE = ref_ext("_gridencoder")
-    if GE is not None:
+    R = refgold.Reference(f"grid_encoder_D{D}_t{gridtype}_i{interp}", GE is not None)
+    if R.live:
         o2 = torch.empty(L, B, C, device="cuda"); dy2 = torch.empty(B, L * D * C, device="cuda")
         GE.grid_encode_forward(cu(x), cu(emb), cu(offsets), o2, B, D, C, L, S, 16, dy2, gridtype, False, interp)
-        if interp == 0:
-            assert torch.equal(o2, out), "grid forward not bit-identical to the compiled reference"
-        else:
-            assert_close(out.cpu().numpy(), o2.cpu().numpy(), rel=1e-6, abs_=1e-7, what="grid fwd (smoothstep) vs reference")
-        assert_close(dy.cpu().numpy(), dy2.cpu().numpy(), rel=1e-5, abs_=1e-4, what="dy_dx vs reference")
+        R.put("out", o2.reshape(-1)); R.put("dy_dx", dy2.reshape(-1))
+    if interp == 0:
+        assert R.equal("out", out.reshape(-1)), "grid forward not bit-identical to the compiled reference"
+    else:
+        assert_close(out.reshape(-1).cpu().numpy()[R.rows("out")], R["out"], rel=1e-6, abs_=1e-7, what="grid fwd (smoothstep) vs reference")
+    assert_close(dy.reshape(-1).cpu().numpy()[R.rows("dy_dx")], R["dy_dx"], rel=1e-5, abs_=1e-4, what="dy_dx vs reference")
     # backward: scatter + input gradient
     grad = np.random.RandomState(40).randn(L, B, C).astype(np.float32)
     gg_ref, gi_ref = oracle_ops.grid_encode_backward(grad, x, emb, offsets, S, 16, dy_ref, gridtype, False, interp)
@@ -346,17 +363,21 @@ def test_sh_and_freq(oracle_ops):
     from geneface_b200 import _lib
     _, d = scenes.field_samples(2048, seed=70)
     SH = ref_ext("_shencoder")
+    R = refgold.Reference("sh_freq", SH is not None)
     for deg in range(1, 9):
         out_ref, dy_ref = oracle_ops.sh_encode_forward(d, deg, True)
         out = torch.empty(2048, deg * deg, device="cuda"); dy = torch.empty(2048, 3 * deg * deg, device="cuda")
         _lib.check(_lib.lib().gf_sh_encode_forward(_lib.ptr(cu(d)), _lib.ptr(out), 2048, 3, deg, _lib.ptr(dy), _lib.stream_ptr()))
         assert_close(out.cpu().numpy(), out_ref, rel=1e-4, abs_=2e-5, what=f"sh deg {deg}")
         assert_close(dy.cpu().numpy(), dy_ref, rel=1e-4, abs_=2e-4, what=f"sh dy_dx deg {deg}")
-        if SH is not None:
+        if R.live:
             o2 = torch.empty(2048, deg * deg, device="cuda"); dy2 = torch.empty(2048, 3 * deg * deg, device="cuda")
             SH.sh_encode_forward(cu(d), o2, 2048, 3, deg, dy2)
-            assert_close(out.cpu().numpy(), o2.cpu().numpy(), rel=1e-4, abs_=2e-5, what=f"sh deg {deg} vs reference")
-            assert_close(dy.cpu().numpy(), dy2.cpu().numpy(), rel=1e-4, abs_=2e-4, what=f"sh dy_dx deg {deg} vs reference")
+            for k, v in ((f"sh_{deg}", o2), (f"sh_dy_dx_{deg}", dy2)):
+                R.put(k, v.reshape(-1), rows=np.random.RandomState(deg).choice(v.numel(), 256, replace=False))
+        assert_close(out.reshape(-1).cpu().numpy()[R.rows(f"sh_{deg}")], R[f"sh_{deg}"], rel=1e-4, abs_=2e-5, what=f"sh deg {deg} vs reference")
+        assert_close(dy.reshape(-1).cpu().numpy()[R.rows(f"sh_dy_dx_{deg}")], R[f"sh_dy_dx_{deg}"], rel=1e-4, abs_=2e-4,
+                     what=f"sh dy_dx deg {deg} vs reference")
     rs = np.random.RandomState(80)
     from geneface_b200.encoders import FreqEncoder
     for D, deg, x in ((6, 4, (rs.randn(64, 6) * 1.5).astype(np.float32)), (2, 10, (rs.rand(4096, 2) * 2 - 1).astype(np.float32))):
@@ -369,10 +390,11 @@ def test_sh_and_freq(oracle_ops):
         (y * cu(g)).sum().backward()
         assert_close(xt.grad.cpu().numpy(), oracle_ops.freq_encode_backward(g, ref, deg, D), rel=2e-3, abs_=0.5, what="freq bwd")
         FQ = ref_ext("_freqencoder")
-        if FQ is not None:
+        if R.live:
             o2 = torch.empty_like(y)
             FQ.freq_encode_forward(cu(x), x.shape[0], D, deg, enc.output_dim, o2)
-            assert torch.equal(o2, y.detach()), "freq forward not bit-identical to the compiled reference"
+            R.put(f"freq_{D}_{deg}", o2, rows="digest")
+        assert R.equal(f"freq_{D}_{deg}", y.detach()), "freq forward not bit-identical to the compiled reference"
 
 
 # ------------------------------------------------------------------------------------------------ field + frame
@@ -459,23 +481,28 @@ def test_fused_frame_vs_cpu_oracle(bitfield, sigma_scale, Himg):
 def test_fused_frame_vs_compiled_reference_renderer(torso, bitfield, sigma_scale):
     """128x128 frame against the reference renderer assembled from the compiled reference kernels (oracle/_ref)."""
     from oracle import ref_gpu
-    if not ref_gpu.available():
-        pytest.skip("oracle/_ref not built")
     from geneface_b200 import synthetic, utils
     Himg = 128
+    N = Himg * Himg
     model, hp = synthetic.build_model(torso=torso, bitfield=bitfield, seed=4, sigma_scale=sigma_scale)
     fi = synthetic.frame_inputs(Himg, Himg)
     rays = utils.get_rays(fi['pose'], fi['intrinsics'], Himg, Himg)
     bg_coords = utils.get_bg_coords(Himg, Himg, 'cuda')
-    ref = ref_gpu.RefRenderer(model.state_dict(), hp, torso=torso)
+    R = refgold.Reference(f"ref_renderer_{'torso' if torso else 'head'}_{bitfield}_{sigma_scale:g}", ref_gpu.available())
     with torch.no_grad():
         cond_feat = model.cal_cond_feat(fi['cond'])
-        trace = []
-        ws, depth, img, nears, fars, _ = ref.render_head(rays['rays_o'][0], rays['rays_d'][0], cond_feat, hp['dt_gamma'], hp['max_steps'], trace=trace)
-        bg = fi['bg_color'][0]
-        if torso:
-            bg, t_alpha, mask = ref.torso_bg(bg_coords[0], fi['poses6'], bg)
-        img_r, depth_r = ref.finish(img, ws, depth, nears, fars, bg)
+        if R.live:
+            ref = ref_gpu.RefRenderer(model.state_dict(), hp, torso=torso)
+            trace = []
+            ws, depth, img, nears, fars, _ = ref.render_head(rays['rays_o'][0], rays['rays_d'][0], cond_feat, hp['dt_gamma'], hp['max_steps'], trace=trace)
+            bg = fi['bg_color'][0]
+            if torso:
+                bg, t_alpha, mask = ref.torso_bg(bg_coords[0], fi['poses6'], bg)
+                R.put("torso_alpha", t_alpha.reshape(N, -1)); R.put("torso_rgb", bg.reshape(N, -1)); R.put("torso_pixels", mask.sum())
+            img_r, depth_r = ref.finish(img, ws, depth, nears, fars, bg)
+            R.put("trace", trace)
+            for k, v in (("rgb_map", img_r), ("depth_map", depth_r), ("weights_sum", ws)):
+                R.put(k, v.reshape(N, -1))
         # (1) through the drop-in render() boundary with explicit rays
         res = model.render(rays['rays_o'], rays['rays_d'], fi['cond'], bg_coords, fi['poses6'], bg_color=fi['bg_color'], **hp)
         # (2) through the pose/intrinsics fast path (in-kernel ray generation), with the termination histogram
@@ -484,17 +511,20 @@ def test_fused_frame_vs_compiled_reference_renderer(torso, bitfield, sigma_scale
                                  want=('weights_sum', 'term_hist') + (('torso_alpha_map', 'torso_rgb_map') if torso else ()))
     # same rays as the reference -> the reference host loop's (n_alive, n_step) sequence must be reproduced exactly
     tr, s_total = replay_schedule(res['term_hist'].cpu().numpy(), Himg * Himg, hp['max_steps'])
-    assert tr == trace, f"reference host loop (n_alive, n_step) sequence differs:\n ours {tr}\n ref  {trace}"
-    assert_close(res['rgb_map'][0].cpu().numpy(), img_r.cpu().numpy(), what="rgb_map (render())")
-    assert_close(res['depth_map'][0].cpu().numpy(), depth_r.cpu().numpy(), what="depth_map (render())")
-    assert_close(res['weights_sum_eval'].cpu().numpy(), ws.cpu().numpy(), what="weights_sum (render())")
+    assert tr == R["trace"], f"reference host loop (n_alive, n_step) sequence differs:\n ours {tr}\n ref  {R['trace']}"
+
+    def vs_ref(ours, key, what):
+        assert_close(ours.reshape(N, -1).cpu().numpy()[R.rows(key)], R[key], what=what)
+    vs_ref(res['rgb_map'][0], "rgb_map", "rgb_map (render())")
+    vs_ref(res['depth_map'][0], "depth_map", "depth_map (render())")
+    vs_ref(res['weights_sum_eval'], "weights_sum", "weights_sum (render())")
     if bitfield == 'S' and sigma_scale <= 4:     # in-kernel ray generation differs from torch's get_rays by <= 1 ulp: only meaningful on a smooth occupancy
-        assert_close(out['rgb_map'].cpu().numpy(), img_r.cpu().numpy(), what="rgb_map (in-kernel rays)")
-        assert_close(out['weights_sum'].cpu().numpy(), ws.cpu().numpy(), what="weights_sum (in-kernel rays)")
+        vs_ref(out['rgb_map'], "rgb_map", "rgb_map (in-kernel rays)")
+        vs_ref(out['weights_sum'], "weights_sum", "weights_sum (in-kernel rays)")
     if torso:
-        assert_close(out['torso_alpha_map'].cpu().numpy(), t_alpha[:, 0].cpu().numpy(), what="torso_alpha")
-        assert_close(out['torso_rgb_map'].cpu().numpy(), bg.cpu().numpy(), what="torso_rgb_map")
-        assert int(mask.sum()) > 0
+        vs_ref(out['torso_alpha_map'], "torso_alpha", "torso_alpha")
+        vs_ref(out['torso_rgb_map'], "torso_rgb", "torso_rgb_map")
+        assert int(R["torso_pixels"]) > 0
 
 
 def test_fused_equals_reference_loop_mode_and_is_deterministic(head_model):
@@ -744,15 +774,19 @@ def test_get_rays_operator_vs_oracle_and_the_reference():
     ro, rd = OF.get_rays(fi['pose'][0].cpu().numpy(), fi['intrinsics'], H, W)
     assert np.abs(r['rays_d'][0].cpu().numpy() - rd).max() < 3e-7 and np.array_equal(r['rays_o'][0].cpu().numpy(), ro)
     assert r['inds'].shape == (1, H * W) and torch.equal(r['inds'][0].cpu(), torch.arange(H * W))
-    if not ref_model.available():
-        return
-    ns = ref_model.load()
+    R = refgold.Reference("get_rays", ref_model.available())
     poses = torch.cat([fi['pose'], synthetic.frame_inputs(H, W, yaw_deg=-3.0)['pose']])
-    for kw in (dict(), dict(N=500), dict(N=640, patch_size=8), dict(rect=(4, 20, 10, 40))):
+    for n, kw in enumerate((dict(), dict(N=500), dict(N=640, patch_size=8), dict(rect=(4, 20, 10, 40)))):
         torch.manual_seed(5)
         a = utils.get_rays(poses, fi['intrinsics'], H, W, **kw)
-        torch.manual_seed(5)
-        b = ns.utils.get_rays(poses, fi['intrinsics'], H, W, **kw)
+        if R.live:
+            torch.manual_seed(5)
+            b = ref_model.load().utils.get_rays(poses, fi['intrinsics'], H, W, **kw)
+            for k in ('inds', 'i', 'j'):
+                R.put(f"{n}/{k}", b[k][0].float(), rows="digest")
+            R.put(f"{n}/rays_o", b['rays_o'].contiguous(), rows="digest")
+            R.put(f"{n}/rays_d", b['rays_d'].reshape(-1, 3))
         for k in ('inds', 'i', 'j'):                   # the reference expands these over the batch in some modes only: compare pose 0
-            assert torch.equal(a[k][0].float(), b[k][0].float()), (k, kw)
-        assert torch.equal(a['rays_o'], b['rays_o'].contiguous()) and (a['rays_d'] - b['rays_d']).abs().max().item() < 3e-7, kw
+            assert R.equal(f"{n}/{k}", a[k][0].float()), (k, kw)
+        rows = R.rows(f"{n}/rays_d")
+        assert R.equal(f"{n}/rays_o", a['rays_o']) and np.abs(a['rays_d'].reshape(-1, 3).cpu().numpy()[rows] - R[f"{n}/rays_d"]).max() < 3e-7, kw
