@@ -199,6 +199,8 @@ __device__ __forceinline__ uint32_t sp_setup(uint8_t* smem, uint32_t sbase, cons
 // z+1 plane only when it exists.  Interpolation is bilinear per z-plane, then a lerp in z (the fp32 result differs from the
 // reference's corner-order sum by rounding only; it is rounded to fp16 right after).
 // ALLFLAT: every level of the batch drops z and is not hashed -> only the 4 corners of the z0 plane exist (uniform fast path).
+// NOWRAP: every level of the batch is dense and its corner indices stay below its size (GridLevels::nowrap), so the mask is a no-op and the
+// corners are rows of 2 adjacent entries: one address per row, the +1 corner an immediate offset of the load (uniform fast path).
 // floor() of a grid coordinate without the conversion pipe.  p = x * scale + 0.5 lies in [0.5, 2^23): adding 2^23 with round-toward-minus-infinity
 // leaves floor(p) in the mantissa, exactly; the integer is the low 23 bits and the float is recovered by an exact subtraction.  Replaces F2I.FLOOR +
 // I2F (two conversion-pipe instructions, ~4x the issue cost and ~3x the latency of an FADD, in front of every level's dependent address chain) by
@@ -210,104 +212,160 @@ __device__ __forceinline__ uint32_t sp_setup(uint8_t* smem, uint32_t sbase, cons
 #ifndef GF_FAST_FLOOR
 #define GF_FAST_FLOOR 1
 #endif
-__device__ __forceinline__ uint32_t floor_split(float& p) {
+__device__ __forceinline__ void floor_split2(float2& p, uint32_t (&g)[2]) {
 #if GF_FAST_FLOOR
-    const float t = __fadd_rd(p, 8388608.0f);
-    p = __fsub_rn(p, __fsub_rn(t, 8388608.0f));
-    return __float_as_uint(t) & 0x7fffffu;
+    const float2 t = fadd2_rm(p, bcast2(8388608.0f));
+    p = fsub2(p, fsub2(t, bcast2(8388608.0f)));
+    g[0] = __float_as_uint(t.x) & 0x7fffffu;
+    g[1] = __float_as_uint(t.y) & 0x7fffffu;
 #else
-    const uint32_t g = (uint32_t)floorf(p);
-    p = __fsub_rn(p, (float)g);
-    return g;
+    g[0] = (uint32_t)floorf(p.x); g[1] = (uint32_t)floorf(p.y);
+    p = fsub2(p, make_float2((float)g[0], (float)g[1]));
 #endif
 }
+// v * v * (3 - 2 v) on both lanes, in the scalar smooth_'s order
+__device__ __forceinline__ float2 smooth2(float2 v) { return fmul2(fmul2(v, v), fsub2(bcast2(3.0f), fadd2(v, v))); }
 
-template <bool ALLFLAT>
+// The per-level coordinate arithmetic runs on LEVEL PAIRS (lane 0 = level l, lane 1 = level l + 1) in packed fp32, and the interpolation on
+// CHANNEL PAIRS (both channels of a corner share its weight, which is broadcast to the two lanes): every lane performs the same IEEE
+// operations in the same order as the scalar form, so the features are bit-identical to it.
+template <bool ALLFLAT, bool NOWRAP>
 __device__ __forceinline__ void gather3_dyn4(const GridDesc& g, int l0, float x, float y, float z, float2 (&out)[4]) {
-    float fx[4], fy[4], fz[4];
+    float2 fx[2], fy[2], fz[2];           // fractional coordinates of levels (l0 + 2k, l0 + 2k + 1)
     float2 v[4][8];
     #pragma unroll
-    for (int i = 0; i < 4; i++) {
-        const int l = l0 + i;
-        const float scale = g.lv.scale[l];
-        float px = __fmaf_rn(x, scale, 0.5f), py = __fmaf_rn(y, scale, 0.5f), pz = __fmaf_rn(z, scale, 0.5f);
-        const uint32_t gx = floor_split(px), gy = floor_split(py), gz = floor_split(pz);
-        if (!GF_ASSUME_LINEAR && g.interp == 1) { px = smooth_(px); py = smooth_(py); pz = smooth_(pz); }
-        fx[i] = px; fy[i] = py; fz[i] = pz;
-        const float2* __restrict__ tab = g.lbase[l];
-        const uint32_t mask = g.lv.mask[l], sy = g.lv.sy[l], sz = g.lv.sz[l];
-        const bool hashed = !ALLFLAT && g.lv.hashed[l] != 0;
-        const bool has_z = !ALLFLAT && (hashed || sz != 0);
-        uint32_t idx[8];
-        if (ALLFLAT) {
-            const uint32_t b = gx + gy * sy;
-            idx[0] = b; idx[1] = b + 1; idx[2] = b + sy; idx[3] = b + sy + 1;
-            idx[4] = idx[5] = idx[6] = idx[7] = 0;
-        } else if (hashed) {
-            const uint32_t y0 = gy * HASH_P1, y1 = y0 + HASH_P1, z0 = gz * HASH_P2, z1 = z0 + HASH_P2;
-            idx[0] = gx ^ y0 ^ z0; idx[1] = (gx + 1) ^ y0 ^ z0; idx[2] = gx ^ y1 ^ z0; idx[3] = (gx + 1) ^ y1 ^ z0;
-            idx[4] = gx ^ y0 ^ z1; idx[5] = (gx + 1) ^ y0 ^ z1; idx[6] = gx ^ y1 ^ z1; idx[7] = (gx + 1) ^ y1 ^ z1;
-        } else {
-            const uint32_t b = gx + gy * sy + gz * sz;
-            idx[0] = b; idx[1] = b + 1; idx[2] = b + sy; idx[3] = b + sy + 1;
-            idx[4] = b + sz; idx[5] = b + sz + 1; idx[6] = b + sz + sy; idx[7] = b + sz + sy + 1;
-        }
+    for (int k = 0; k < 2; k++) {
+        const int l = l0 + 2 * k;
+        const float2 scale = make_float2(g.lv.scale[l], g.lv.scale[l + 1]);
+        float2 px = ffma2(bcast2(x), scale, bcast2(0.5f)), py = ffma2(bcast2(y), scale, bcast2(0.5f)), pz = ffma2(bcast2(z), scale, bcast2(0.5f));
+        uint32_t gx[2], gy[2], gz[2];
+        floor_split2(px, gx); floor_split2(py, gy); floor_split2(pz, gz);
+        if (!GF_ASSUME_LINEAR && g.interp == 1) { px = smooth2(px); py = smooth2(py); pz = smooth2(pz); }
         #pragma unroll
-        for (int c = 0; c < 4; c++) v[i][c] = __ldg(tab + (idx[c] & mask));
-        if (!ALLFLAT) {
+        for (int h = 0; h < 2; h++) {
+            const int i = 2 * k + h;
+            const float2* __restrict__ tab = g.lbase[l + h];
+            const uint32_t mask = g.lv.mask[l + h], sy = g.lv.sy[l + h], sz = g.lv.sz[l + h];
+            const bool hashed = !ALLFLAT && !NOWRAP && g.lv.hashed[l + h] != 0;
+            const bool has_z = !ALLFLAT && (hashed || sz != 0);
+            if (NOWRAP) {
+                const float2* __restrict__ r0 = tab + (ALLFLAT ? gx[h] + gy[h] * sy : gx[h] + gy[h] * sy + gz[h] * sz);
+                const float2* __restrict__ r1 = r0 + sy;
+                v[i][0] = __ldg(r0); v[i][1] = __ldg(r0 + 1); v[i][2] = __ldg(r1); v[i][3] = __ldg(r1 + 1);
+                if (!ALLFLAT) {
+                    v[i][4] = has_z ? __ldg(r0 + sz) : make_float2(0.f, 0.f); v[i][5] = has_z ? __ldg(r0 + sz + 1) : make_float2(0.f, 0.f);
+                    v[i][6] = has_z ? __ldg(r1 + sz) : make_float2(0.f, 0.f); v[i][7] = has_z ? __ldg(r1 + sz + 1) : make_float2(0.f, 0.f);
+                    if (!has_z) { if (h == 0) pz.x = 0.f; else pz.y = 0.f; }
+                }
+                continue;
+            }
+            uint32_t idx[8];
+            if (ALLFLAT) {
+                const uint32_t b = gx[h] + gy[h] * sy;
+                idx[0] = b; idx[1] = b + 1; idx[2] = b + sy; idx[3] = b + sy + 1;
+                idx[4] = idx[5] = idx[6] = idx[7] = 0;
+            } else if (hashed) {
+                const uint32_t y0 = gy[h] * HASH_P1, y1 = y0 + HASH_P1, z0 = gz[h] * HASH_P2, z1 = z0 + HASH_P2;
+                const uint32_t x0 = gx[h], x1 = gx[h] + 1;
+                idx[0] = x0 ^ y0 ^ z0; idx[1] = x1 ^ y0 ^ z0; idx[2] = x0 ^ y1 ^ z0; idx[3] = x1 ^ y1 ^ z0;
+                idx[4] = x0 ^ y0 ^ z1; idx[5] = x1 ^ y0 ^ z1; idx[6] = x0 ^ y1 ^ z1; idx[7] = x1 ^ y1 ^ z1;
+            } else {
+                const uint32_t b = gx[h] + gy[h] * sy + gz[h] * sz;
+                idx[0] = b; idx[1] = b + 1; idx[2] = b + sy; idx[3] = b + sy + 1;
+                idx[4] = b + sz; idx[5] = b + sz + 1; idx[6] = b + sz + sy; idx[7] = b + sz + sy + 1;
+            }
             #pragma unroll
-            for (int c = 4; c < 8; c++) v[i][c] = has_z ? __ldg(tab + (idx[c] & mask)) : make_float2(0.f, 0.f);
-            if (!has_z) fz[i] = 0.f;
+            for (int c = 0; c < 4; c++) v[i][c] = __ldg(tab + (idx[c] & mask));
+            if (!ALLFLAT) {
+                #pragma unroll
+                for (int c = 4; c < 8; c++) v[i][c] = has_z ? __ldg(tab + (idx[c] & mask)) : make_float2(0.f, 0.f);
+                if (!has_z) { if (h == 0) pz.x = 0.f; else pz.y = 0.f; }
+            }
         }
+        fx[k] = px; fy[k] = py; fz[k] = pz;
     }
     #pragma unroll
-    for (int i = 0; i < 4; i++) {
-        const float px = fx[i], py = fy[i], pz = fz[i];
-        const float qx = 1.0f - px, qy = 1.0f - py;
-        const float w00 = qx * qy, w10 = px * qy, w01 = qx * py, w11 = px * py;
-        const float a0 = fmaf(w11, v[i][3].x, fmaf(w01, v[i][2].x, fmaf(w10, v[i][1].x, w00 * v[i][0].x)));
-        const float a1 = fmaf(w11, v[i][3].y, fmaf(w01, v[i][2].y, fmaf(w10, v[i][1].y, w00 * v[i][0].y)));
-        if (ALLFLAT) { out[i] = make_float2(a0, a1); continue; }
-        const float b0 = fmaf(w11, v[i][7].x, fmaf(w01, v[i][6].x, fmaf(w10, v[i][5].x, w00 * v[i][4].x)));
-        const float b1 = fmaf(w11, v[i][7].y, fmaf(w01, v[i][6].y, fmaf(w10, v[i][5].y, w00 * v[i][4].y)));
-        out[i] = make_float2(fmaf(pz, b0 - a0, a0), fmaf(pz, b1 - a1, a1));
+    for (int k = 0; k < 2; k++) {
+        const float2 qx = fsub2(bcast2(1.0f), fx[k]), qy = fsub2(bcast2(1.0f), fy[k]);
+        const float2 w00 = fmul2(qx, qy), w10 = fmul2(fx[k], qy), w01 = fmul2(qx, fy[k]), w11 = fmul2(fx[k], fy[k]);
+        #pragma unroll
+        for (int h = 0; h < 2; h++) {
+            const int i = 2 * k + h;
+            const float a00 = h ? w00.y : w00.x, a10 = h ? w10.y : w10.x, a01 = h ? w01.y : w01.x, a11 = h ? w11.y : w11.x;
+            const float2 a = ffma2(bcast2(a11), v[i][3], ffma2(bcast2(a01), v[i][2], ffma2(bcast2(a10), v[i][1], fmul2(bcast2(a00), v[i][0]))));
+            if (ALLFLAT) { out[i] = a; continue; }
+            const float2 b = ffma2(bcast2(a11), v[i][7], ffma2(bcast2(a01), v[i][6], ffma2(bcast2(a10), v[i][5], fmul2(bcast2(a00), v[i][4]))));
+            out[i] = ffma2(bcast2(h ? fz[k].y : fz[k].x), fsub2(b, a), a);
+        }
     }
 }
 
-// 2-D ambient grid, 8 consecutive levels from l0 (32 gathers in flight)
+// 1 when the n levels from l0 are all GridLevels::nowrap (uniform: level constants)
+__device__ __forceinline__ bool levels_nowrap(const GridLevels& lv, int l0, int n) {
+    bool nw = true;
+    #pragma unroll
+    for (int q = 0; q < n; q++) nw = nw && lv.nowrap[l0 + q] != 0;
+    return nw;
+}
+// unit u (levels 4u..4u+3) of the 3-D grid, with the batch's uniform ALLFLAT / NOWRAP properties
+__device__ __forceinline__ void gather3_unit(const GridDesc& g, uint32_t u, bool flat, bool nowrap, float x, float y, float z, float2 (&out)[4]) {
+    if (flat) {
+        if (nowrap) gather3_dyn4<true, true>(g, 4 * u, x, y, z, out);
+        else gather3_dyn4<true, false>(g, 4 * u, x, y, z, out);
+    } else {
+        if (nowrap) gather3_dyn4<false, true>(g, 4 * u, x, y, z, out);
+        else gather3_dyn4<false, false>(g, 4 * u, x, y, z, out);
+    }
+}
+
+// 2-D ambient grid, 8 consecutive levels from l0 (32 gathers in flight); level pairs, channel pairs and NOWRAP as in gather3_dyn4
+template <bool NOWRAP>
 __device__ __forceinline__ void gather2_dyn8(const GridDesc& g, int l0, float x, float y, float2 (&out)[8]) {
     const bool oob = x < 0 || x > 1 || y < 0 || y > 1;            // tanh output mapped to [0,1]: cannot happen, kept for safety
     if (oob) { x = 0.5f; y = 0.5f; }
-    float fx[8], fy[8];
+    float2 fx[4], fy[4];
     float2 v[8][4];
     #pragma unroll
-    for (int i = 0; i < 8; i++) {
-        const int l = l0 + i;
-        const float scale = g.lv.scale[l];
-        float px = __fmaf_rn(x, scale, 0.5f), py = __fmaf_rn(y, scale, 0.5f);
-        const uint32_t gx = floor_split(px), gy = floor_split(py);
-        if (!GF_ASSUME_LINEAR && g.interp == 1) { px = smooth_(px); py = smooth_(py); }
-        fx[i] = px; fy[i] = py;
-        const float2* __restrict__ tab = g.lbase[l];
-        const uint32_t mask = g.lv.mask[l], sy = g.lv.sy[l];
-        uint32_t idx[4];
-        if (g.lv.hashed[l]) {
-            const uint32_t y0 = gy * HASH_P1, y1 = y0 + HASH_P1;
-            idx[0] = gx ^ y0; idx[1] = (gx + 1) ^ y0; idx[2] = gx ^ y1; idx[3] = (gx + 1) ^ y1;
-        } else {
-            const uint32_t b = gx + gy * sy;
-            idx[0] = b; idx[1] = b + 1; idx[2] = b + sy; idx[3] = b + sy + 1;
-        }
+    for (int k = 0; k < 4; k++) {
+        const int l = l0 + 2 * k;
+        const float2 scale = make_float2(g.lv.scale[l], g.lv.scale[l + 1]);
+        float2 px = ffma2(bcast2(x), scale, bcast2(0.5f)), py = ffma2(bcast2(y), scale, bcast2(0.5f));
+        uint32_t gx[2], gy[2];
+        floor_split2(px, gx); floor_split2(py, gy);
+        if (!GF_ASSUME_LINEAR && g.interp == 1) { px = smooth2(px); py = smooth2(py); }
+        fx[k] = px; fy[k] = py;
         #pragma unroll
-        for (int c = 0; c < 4; c++) v[i][c] = __ldg(tab + (idx[c] & mask));
+        for (int h = 0; h < 2; h++) {
+            const float2* __restrict__ tab = g.lbase[l + h];
+            const uint32_t mask = g.lv.mask[l + h], sy = g.lv.sy[l + h];
+            if (NOWRAP) {
+                const float2* __restrict__ r0 = tab + (gx[h] + gy[h] * sy), * __restrict__ r1 = r0 + sy;
+                v[2 * k + h][0] = __ldg(r0); v[2 * k + h][1] = __ldg(r0 + 1); v[2 * k + h][2] = __ldg(r1); v[2 * k + h][3] = __ldg(r1 + 1);
+                continue;
+            }
+            uint32_t idx[4];
+            if (g.lv.hashed[l + h]) {
+                const uint32_t y0 = gy[h] * HASH_P1, y1 = y0 + HASH_P1;
+                idx[0] = gx[h] ^ y0; idx[1] = (gx[h] + 1) ^ y0; idx[2] = gx[h] ^ y1; idx[3] = (gx[h] + 1) ^ y1;
+            } else {
+                const uint32_t b = gx[h] + gy[h] * sy;
+                idx[0] = b; idx[1] = b + 1; idx[2] = b + sy; idx[3] = b + sy + 1;
+            }
+            #pragma unroll
+            for (int c = 0; c < 4; c++) v[2 * k + h][c] = __ldg(tab + (idx[c] & mask));
+        }
     }
     #pragma unroll
-    for (int i = 0; i < 8; i++) {
-        const float px = fx[i], py = fy[i], qx = 1.0f - px, qy = 1.0f - py;
-        const float w00 = qx * qy, w10 = px * qy, w01 = qx * py, w11 = px * py;
-        const float a0 = fmaf(w11, v[i][3].x, fmaf(w01, v[i][2].x, fmaf(w10, v[i][1].x, w00 * v[i][0].x)));
-        const float a1 = fmaf(w11, v[i][3].y, fmaf(w01, v[i][2].y, fmaf(w10, v[i][1].y, w00 * v[i][0].y)));
-        out[i] = oob ? make_float2(0.f, 0.f) : make_float2(a0, a1);
+    for (int k = 0; k < 4; k++) {
+        const float2 qx = fsub2(bcast2(1.0f), fx[k]), qy = fsub2(bcast2(1.0f), fy[k]);
+        const float2 w00 = fmul2(qx, qy), w10 = fmul2(fx[k], qy), w01 = fmul2(qx, fy[k]), w11 = fmul2(fx[k], fy[k]);
+        #pragma unroll
+        for (int h = 0; h < 2; h++) {
+            const int i = 2 * k + h;
+            const float a00 = h ? w00.y : w00.x, a10 = h ? w10.y : w10.x, a01 = h ? w01.y : w01.x, a11 = h ? w11.y : w11.x;
+            const float2 a = ffma2(bcast2(a11), v[i][3], ffma2(bcast2(a01), v[i][2], ffma2(bcast2(a10), v[i][1], fmul2(bcast2(a00), v[i][0]))));
+            out[i] = oob ? make_float2(0.f, 0.f) : a;
+        }
     }
 }
 
@@ -337,13 +395,14 @@ __global__ void __launch_bounds__(SPA_THREADS, 1) k_tc_amb(const SpArgs a) {
         asm volatile("setmaxnreg.inc.sync.aligned.u32 112;");
 #endif
         const uint32_t half = tid >> 7, row = tid & 127;     // half = producer warpgroup 0 .. SPA_PROD_WG-1
-        uint32_t flat_units = 0;          // bit u: levels 4u..4u+3 all drop z and are not hashed
+        uint32_t flat_units = 0, nowrap_units = 0;     // bit u: levels 4u..4u+3 all drop z and are not hashed / are all nowrap
         #pragma unroll
         for (int u = 0; u < 4; u++) {
             bool flat = true;
             #pragma unroll
             for (int q = 0; q < 4; q++) flat = flat && a.grid.lv.sz[4 * u + q] == 0 && a.grid.lv.hashed[4 * u + q] == 0;
             flat_units |= (flat ? 1u : 0u) << u;
+            nowrap_units |= (levels_nowrap(a.grid.lv, 4 * u, 4) ? 1u : 0u) << u;
         }
         // This warpgroup's units (4 levels each) of a row.  Two warpgroups: u = wg and wg + 2 (one 8-corner coarse unit + one z-dropped fine unit
         // each).  Three: the cheapest pair of units (cost 2 per 8-corner unit, 1 per z-dropped one) shares a warpgroup, the other two units get one each.
@@ -403,13 +462,12 @@ __global__ void __launch_bounds__(SPA_THREADS, 1) k_tc_amb(const SpArgs a) {
             for (uint32_t b = 0; b < my_nu; b++) {
                 const uint32_t u = b == 0 ? my_u0 : my_u1;
                 float2 f[4];
-                if ((flat_units >> u) & 1) gather3_dyn4<true>(a.grid, 4 * u, ux, uy, uz, f);
-                else gather3_dyn4<false>(a.grid, 4 * u, ux, uy, uz, f);
+                gather3_unit(a.grid, u, (flat_units >> u) & 1, (nowrap_units >> u) & 1, ux, uy, uz, f);
                 if (oob) { f[0] = f[1] = f[2] = f[3] = make_float2(0.f, 0.f); }
-                const uint4 hi = make_uint4(pack_h2(f[0].x, f[0].y), pack_h2(f[1].x, f[1].y), pack_h2(f[2].x, f[2].y), pack_h2(f[3].x, f[3].y));
+                uint4 hi, lo;
+                pack_hilo_h2(f[0], hi.x, lo.x); pack_hilo_h2(f[1], hi.y, lo.y); pack_hilo_h2(f[2], hi.z, lo.z); pack_hilo_h2(f[3], hi.w, lo.w);
                 sts128(F + sw128(row, u), hi);
-                sts128(F + sw128(row, 4 + u), make_uint4(pack_h2(h_resid(f[0].x), h_resid(f[0].y)), pack_h2(h_resid(f[1].x), h_resid(f[1].y)),
-                                                         pack_h2(h_resid(f[2].x), h_resid(f[2].y)), pack_h2(h_resid(f[3].x), h_resid(f[3].y))));
+                sts128(F + sw128(row, 4 + u), lo);
                 if (b == 0) keep0 = hi; else keep1 = hi;
                 if (row == 0 && half < 2) TT_STAMP(0, 2 + half, j, 2 + b);
                 if (row == 0 && half < 2 && my_nu == 1) TT_STAMP(0, 2 + half, j, 3);
@@ -569,6 +627,7 @@ __global__ void __launch_bounds__(SP_THREADS, 1) k_tc_sigcol(const SpArgs a) {
     if (warp < 8) {
         // ------------------------------------------------ producers ------------------------------------------------
         const uint32_t half = tid >> 7, row = tid & 127;
+        const bool nowrap_half = levels_nowrap(a.grid.lv, 8 * half, 8);
         // Per-row inputs of a tile (32 B of position features, the ambient coordinate, the ray's view direction) are staged ONE TILE AHEAD with
         // cp.async -- the features and the direction straight into the NEXT ring slot, which is therefore acquired one tile early -- and the ray
         // id TWO tiles ahead, so that the dependent pos4.w -> rays_d chain never sits on a producer's critical path.  (As register prefetches the
@@ -625,7 +684,8 @@ __global__ void __launch_bounds__(SP_THREADS, 1) k_tc_sigcol(const SpArgs a) {
             }
             const float vx = (ap.x + 1.0f) * 0.5f, vy = (ap.y + 1.0f) * 0.5f;
             float2 f[8];
-            gather2_dyn8(a.grid, 8 * half, vx, vy, f);
+            if (nowrap_half) gather2_dyn8<true>(a.grid, 8 * half, vx, vy, f);
+            else gather2_dyn8<false>(a.grid, 8 * half, vx, vy, f);
             #pragma unroll
             for (int u = 0; u < 2; u++)
                 sts128(F + sw128(row, 4 + 2 * half + u), make_uint4(pack_h2(f[4 * u].x, f[4 * u].y), pack_h2(f[4 * u + 1].x, f[4 * u + 1].y),
@@ -795,7 +855,8 @@ __global__ void __launch_bounds__(256) k_gather_probe(GridDesc pos, GridDesc amb
                                                       const float2* __restrict__ amb_pos, uint32_t M, float2* __restrict__ out) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= M) return;
-    const float ux = (xyzs[3 * (size_t)i] + bound) * inv2b, uy = (xyzs[3 * (size_t)i + 1] + bound) * inv2b, uz = (xyzs[3 * (size_t)i + 2] + bound) * inv2b;
+    float ux = (xyzs[3 * (size_t)i] + bound) * inv2b, uy = (xyzs[3 * (size_t)i + 1] + bound) * inv2b, uz = (xyzs[3 * (size_t)i + 2] + bound) * inv2b;
+    if (ux < 0 || ux > 1 || uy < 0 || uy > 1 || uz < 0 || uz > 1) { ux = 0.5f; uy = 0.5f; uz = 0.5f; }     // as the producers: corner indices stay in range
     float2 acc = make_float2(0.f, 0.f);
     #pragma unroll 1
     for (int u = 0; u < 4; u++) {
@@ -803,8 +864,7 @@ __global__ void __launch_bounds__(256) k_gather_probe(GridDesc pos, GridDesc amb
         #pragma unroll
         for (int q = 0; q < 4; q++) flat = flat && pos.lv.sz[4 * u + q] == 0 && pos.lv.hashed[4 * u + q] == 0;
         float2 f[4];
-        if (flat) gather3_dyn4<true>(pos, 4 * u, ux, uy, uz, f);
-        else gather3_dyn4<false>(pos, 4 * u, ux, uy, uz, f);
+        gather3_unit(pos, u, flat, levels_nowrap(pos.lv, 4 * u, 4), ux, uy, uz, f);
         #pragma unroll
         for (int q = 0; q < 4; q++) { acc.x += f[q].x; acc.y += f[q].y; }
     }
@@ -813,7 +873,8 @@ __global__ void __launch_bounds__(256) k_gather_probe(GridDesc pos, GridDesc amb
     #pragma unroll 1
     for (int h = 0; h < 2; h++) {
         float2 f[8];
-        gather2_dyn8(amb, 8 * h, vx, vy, f);
+        if (levels_nowrap(amb.lv, 8 * h, 8)) gather2_dyn8<true>(amb, 8 * h, vx, vy, f);
+        else gather2_dyn8<false>(amb, 8 * h, vx, vy, f);
         #pragma unroll
         for (int q = 0; q < 8; q++) { acc.x += f[q].x; acc.y += f[q].y; }
     }

@@ -21,6 +21,7 @@ struct GridLevels {
     uint32_t sz[16];       // stride of z (0 when dropped; unused for 2-D grids)
     uint32_t mask[16];     // index & mask  ==  index % hsize
     uint32_t hashed[16];   // 1: fast_hash index (gridtype 0 on a clipped level)
+    uint32_t nowrap[16];   // 1: dense level whose largest corner index stays below hsize: the mask never changes an index
 };
 
 struct GridDesc {

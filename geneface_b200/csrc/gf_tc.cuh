@@ -145,12 +145,53 @@ __device__ __forceinline__ uint32_t lds32(uint32_t saddr) {
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
 
+// Packed two-lane fp32 arithmetic (Blackwell FFMA2 / FADD2 / FMUL2): each lane is the same IEEE operation, with the same rounding, as the
+// scalar __fmaf_rn / __fadd_rn / __fsub_rn / __fmul_rn (/ __fadd_rd) on that lane, so replacing a pair of scalar operations by one of these keeps
+// results bit-identical.  The register-pair moves disappear in SASS when ptxas keeps the float2 in an aligned pair; a lane-broadcast first
+// operand (make_float2(w, w)) compiles to the .F32 operand form, without a move.
+__device__ __forceinline__ uint64_t f2_pack(float2 a) {
+    uint64_t r;
+    asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(a.x), "f"(a.y));
+    return r;
+}
+__device__ __forceinline__ float2 f2_unpack(uint64_t r) {
+    float2 d;
+    asm("mov.b64 {%0, %1}, %2;" : "=f"(d.x), "=f"(d.y) : "l"(r));
+    return d;
+}
+// d = a * b + c
+__device__ __forceinline__ float2 ffma2(float2 a, float2 b, float2 c) {
+    uint64_t d;
+    asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(f2_pack(a)), "l"(f2_pack(b)), "l"(f2_pack(c)));
+    return f2_unpack(d);
+}
+__device__ __forceinline__ float2 fadd2(float2 a, float2 b) {
+    uint64_t d;
+    asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(f2_pack(a)), "l"(f2_pack(b)));
+    return f2_unpack(d);
+}
+// rounding toward minus infinity (floor_split2)
+__device__ __forceinline__ float2 fadd2_rm(float2 a, float2 b) {
+    uint64_t d;
+    asm("add.rm.f32x2 %0, %1, %2;" : "=l"(d) : "l"(f2_pack(a)), "l"(f2_pack(b)));
+    return f2_unpack(d);
+}
+__device__ __forceinline__ float2 fsub2(float2 a, float2 b) {
+    uint64_t d;
+    asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(f2_pack(a)), "l"(f2_pack(b)));
+    return f2_unpack(d);
+}
+__device__ __forceinline__ float2 fmul2(float2 a, float2 b) {
+    uint64_t d;
+    asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(f2_pack(a)), "l"(f2_pack(b)));
+    return f2_unpack(d);
+}
+__device__ __forceinline__ float2 bcast2(float w) { return make_float2(w, w); }
+
 __device__ __forceinline__ uint32_t pack_h2(float lo, float hi) {
     const __half2 h = __floats2half2_rn(lo, hi);
     return *reinterpret_cast<const uint32_t*>(&h);
 }
-__device__ __forceinline__ float h_resid(float v) { return v - __half2float(__float2half_rn(v)); }   // the part fp16 drops
-
 
 // ReLU + fp16x2 pack in ONE instruction (cvt.relu): low half = max(lo, 0), high half = max(hi, 0)
 __device__ __forceinline__ uint32_t pack_relu_h2(float lo, float hi) {
@@ -165,6 +206,12 @@ __device__ __forceinline__ uint32_t pack_relu_rz_h2(float lo, float hi) {
     return r;
 }
 __device__ __forceinline__ float2 unpack_h2(uint32_t p) { return __half22float2(*reinterpret_cast<const __half2*>(&p)); }
+// fp16 hi/lo split of two values: hi = rn(f), lo = rn(f - hi) (the part fp16 drops), each packed as fp16x2
+__device__ __forceinline__ void pack_hilo_h2(float2 f, uint32_t& hi, uint32_t& lo) {
+    hi = pack_h2(f.x, f.y);
+    const float2 r = fsub2(f, unpack_h2(hi));
+    lo = pack_h2(r.x, r.y);
+}
 
 // NCHUNK x 32 accumulator columns starting at col0 (this thread's TMEM lane) -> (+bias) -> ReLU -> fp16 -> A operand region.
 // SPLIT: also emit the fp16 residual into a second A region (hi + lo ~ 21-bit operand): hi = rz(relu(v)) so that the
@@ -248,11 +295,15 @@ __device__ __forceinline__ void epilogue_relu_to_A_pipe(uint32_t t_d, uint32_t t
         uint32_t p[16];
         #pragma unroll
         for (int i = 0; i < 16; i += 2) {
-            float v0 = __uint_as_float(cur[2 * i]), v1 = __uint_as_float(cur[2 * i + 1]);
-            float v2 = __uint_as_float(cur[2 * i + 2]), v3 = __uint_as_float(cur[2 * i + 3]);
-            if (BIAS) { const float4 b = lds128(bias_saddr + 4 * (32 * c + 2 * i)); v0 += b.x; v1 += b.y; v2 += b.z; v3 += b.w; }
-            p[i] = pack_relu_h2(v0, v1);
-            p[i + 1] = pack_relu_h2(v2, v3);
+            float2 v01 = make_float2(__uint_as_float(cur[2 * i]), __uint_as_float(cur[2 * i + 1]));
+            float2 v23 = make_float2(__uint_as_float(cur[2 * i + 2]), __uint_as_float(cur[2 * i + 3]));
+            if (BIAS) {
+                const float4 b = lds128(bias_saddr + 4 * (32 * c + 2 * i));
+                v01 = fadd2(v01, make_float2(b.x, b.y));
+                v23 = fadd2(v23, make_float2(b.z, b.w));
+            }
+            p[i] = pack_relu_h2(v01.x, v01.y);
+            p[i + 1] = pack_relu_h2(v23.x, v23.y);
         }
         tmem_st16(t_a + 16 * c, p);
         if (c < 3) tmem_wait_ld32(r[(c + 1) & 1]);
@@ -278,13 +329,13 @@ __device__ __forceinline__ void epilogue_split_to_A_pipe(uint32_t t_d, uint32_t 
         #pragma unroll
         for (int i = 0; i < 16; i += 2) {
             const float4 b = lds128(bias_saddr + 4 * (32 * c + 2 * i));
-            const float v0 = __uint_as_float(cur[2 * i]) + b.x, v1 = __uint_as_float(cur[2 * i + 1]) + b.y;
-            const float v2 = __uint_as_float(cur[2 * i + 2]) + b.z, v3 = __uint_as_float(cur[2 * i + 3]) + b.w;
-            p[i] = pack_relu_rz_h2(v0, v1);
-            p[i + 1] = pack_relu_rz_h2(v2, v3);
-            const float2 h0 = unpack_h2(p[i]), h1 = unpack_h2(p[i + 1]);
-            q[i] = pack_relu_h2(v0 - h0.x, v1 - h0.y);
-            q[i + 1] = pack_relu_h2(v2 - h1.x, v3 - h1.y);
+            const float2 v01 = fadd2(make_float2(__uint_as_float(cur[2 * i]), __uint_as_float(cur[2 * i + 1])), make_float2(b.x, b.y));
+            const float2 v23 = fadd2(make_float2(__uint_as_float(cur[2 * i + 2]), __uint_as_float(cur[2 * i + 3])), make_float2(b.z, b.w));
+            p[i] = pack_relu_rz_h2(v01.x, v01.y);
+            p[i + 1] = pack_relu_rz_h2(v23.x, v23.y);
+            const float2 l01 = fsub2(v01, unpack_h2(p[i])), l23 = fsub2(v23, unpack_h2(p[i + 1]));
+            q[i] = pack_relu_h2(l01.x, l01.y);
+            q[i + 1] = pack_relu_h2(l23.x, l23.y);
         }
         tmem_st16(t_a + 16 * c, p);
         tmem_st16(t_alo + 16 * c, q);
@@ -293,16 +344,5 @@ __device__ __forceinline__ void epilogue_split_to_A_pipe(uint32_t t_d, uint32_t 
     tmem_wait_st();
 }
 
-// packed fp32 FMA (Blackwell FFMA2): d = a * b + c on two lanes
-__device__ __forceinline__ float2 ffma2(float2 a, float2 b, float2 c) {
-    uint64_t ra, rb, rc, rd;
-    asm("mov.b64 %0, {%1, %2};" : "=l"(ra) : "f"(a.x), "f"(a.y));
-    asm("mov.b64 %0, {%1, %2};" : "=l"(rb) : "f"(b.x), "f"(b.y));
-    asm("mov.b64 %0, {%1, %2};" : "=l"(rc) : "f"(c.x), "f"(c.y));
-    asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(rd) : "l"(ra), "l"(rb), "l"(rc));
-    float2 d;
-    asm("mov.b64 {%0, %1}, %2;" : "=f"(d.x), "=f"(d.y) : "l"(rd));
-    return d;
-}
 
 }  // namespace gf

@@ -62,10 +62,9 @@ __global__ void k_level_geometry(const int* __restrict__ offsets, float S, uint3
     out->mask[l] = pow2 ? hs - 1 : 0xFFFFFFFFu;
     // `index % hsize` is only replaced by the mask when it is provably the same: power-of-two level, or a dense level
     // whose largest reachable index (pos_grid <= res per axis) stays below hsize.
-    if (!pow2) {
-        const unsigned long long maxidx = (unsigned long long)res * (1ull + sy + sz);
-        if (out->hashed[l] || maxidx >= hs) *bad = 1;
-    }
+    const unsigned long long maxidx = (unsigned long long)res * (1ull + sy + sz);
+    out->nowrap[l] = (!out->hashed[l] && maxidx < hs) ? 1u : 0u;
+    if (!pow2 && !out->nowrap[l]) *bad = 1;
 }
 
 // dst[k][n] = src[n][k0 + k]   (src row-major [N][ldsrc]); dst row stride ldd

@@ -1,8 +1,9 @@
 #!/usr/bin/env python
 """SASS opcode histogram of the tensor-core kernels of libgfrender.so (CPU only: cuobjdump), the static evidence next to the ncu counters:
-   python scripts/sass_histogram.py > profiles/r02_sass_opcodes.txt
+   python scripts/sass_histogram.py [libgfrender.so] > profiles/r03_sass_opcodes.txt
 Per kernel: instruction count, code bytes, and the opcodes that prove the Blackwell path (UTCHMMA = tcgen05.mma, LDTM/STTM = tcgen05.ld/st,
-UBLKCP = cp.async.bulk (TMA), LDGSTS = cp.async, UTCBAR = tcgen05.commit, SYNCS = mbarrier, ELECT = elect.sync, USETMAXREG = setmaxnreg)."""
+UBLKCP = cp.async.bulk (TMA), LDGSTS = cp.async, UTCBAR = tcgen05.commit, SYNCS = mbarrier, ELECT = elect.sync, USETMAXREG = setmaxnreg),
+and the packed (FFMA2 / FADD2 / FMUL2) next to the scalar fp32 arithmetic."""
 import collections
 import os
 import re
@@ -11,7 +12,7 @@ import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 so = sys.argv[1] if len(sys.argv) > 1 else os.path.join(ROOT, "geneface_b200", "libgfrender.so")
-KEY = ("UTCHMMA", "LDTM", "STTM", "UBLKCP", "LDGSTS", "UTCBAR", "SYNCS", "ELECT", "USETMAXREG", "R2UR", "FFMA2", "F2FP", "LDG", "LDS", "STS", "LD", "ST", "LDC", "ATOMS", "RED", "F2I", "I2FP")
+KEY = ("UTCHMMA", "LDTM", "STTM", "UBLKCP", "LDGSTS", "UTCBAR", "SYNCS", "ELECT", "USETMAXREG", "R2UR", "FFMA2", "FADD2", "FMUL2", "FFMA", "FADD", "FMUL", "HADD2", "F2FP", "LDG", "LDS", "STS", "LD", "ST", "LDC", "ATOMS", "RED", "F2I", "I2FP")
 txt = subprocess.run(["cuobjdump", "-sass", so], capture_output=True, text=True, check=True).stdout
 cur, hist = None, collections.OrderedDict()
 for ln in txt.splitlines():
