@@ -199,8 +199,9 @@ __device__ __forceinline__ uint32_t sp_setup(uint8_t* smem, uint32_t sbase, cons
 // z+1 plane only when it exists.  Interpolation is bilinear per z-plane, then a lerp in z (the fp32 result differs from the
 // reference's corner-order sum by rounding only; it is rounded to fp16 right after).
 // ALLFLAT: every level of the batch drops z and is not hashed -> only the 4 corners of the z0 plane exist (uniform fast path).
-// NOWRAP: every level of the batch is dense and its corner indices stay below its size (GridLevels::nowrap), so the mask is a no-op and the
-// corners are rows of 2 adjacent entries: one address per row, the +1 corner an immediate offset of the load (uniform fast path).
+// CONTIG: no level of the batch is hashed.  The tables are the padded images of GridLevels::pad, so a cell's corners are rows of 2 adjacent
+// entries from the masked base index, on wrapping levels too: one address per row, the +1 corner an immediate offset of the load (uniform fast
+// path).  Only batches with a hashed level compute, mask and address each corner.
 // floor() of a grid coordinate without the conversion pipe.  p = x * scale + 0.5 lies in [0.5, 2^23): adding 2^23 with round-toward-minus-infinity
 // leaves floor(p) in the mantissa, exactly; the integer is the low 23 bits and the float is recovered by an exact subtraction.  Replaces F2I.FLOOR +
 // I2F (two conversion-pipe instructions, ~4x the issue cost and ~3x the latency of an FADD, in front of every level's dependent address chain) by
@@ -229,8 +230,9 @@ __device__ __forceinline__ float2 smooth2(float2 v) { return fmul2(fmul2(v, v), 
 // The per-level coordinate arithmetic runs on LEVEL PAIRS (lane 0 = level l, lane 1 = level l + 1) in packed fp32, and the interpolation on
 // CHANNEL PAIRS (both channels of a corner share its weight, which is broadcast to the two lanes): every lane performs the same IEEE
 // operations in the same order as the scalar form, so the features are bit-identical to it.
-template <bool ALLFLAT, bool NOWRAP>
+template <bool ALLFLAT, bool CONTIG>
 __device__ __forceinline__ void gather3_dyn4(const GridDesc& g, int l0, float x, float y, float z, float2 (&out)[4]) {
+    static_assert(CONTIG || !ALLFLAT, "an ALLFLAT batch has no hashed level");
     float2 fx[2], fy[2], fz[2];           // fractional coordinates of levels (l0 + 2k, l0 + 2k + 1)
     float2 v[4][8];
     #pragma unroll
@@ -246,10 +248,10 @@ __device__ __forceinline__ void gather3_dyn4(const GridDesc& g, int l0, float x,
             const int i = 2 * k + h;
             const float2* __restrict__ tab = g.lbase[l + h];
             const uint32_t mask = g.lv.mask[l + h], sy = g.lv.sy[l + h], sz = g.lv.sz[l + h];
-            const bool hashed = !ALLFLAT && !NOWRAP && g.lv.hashed[l + h] != 0;
+            const bool hashed = !CONTIG && g.lv.hashed[l + h] != 0;
             const bool has_z = !ALLFLAT && (hashed || sz != 0);
-            if (NOWRAP) {
-                const float2* __restrict__ r0 = tab + (ALLFLAT ? gx[h] + gy[h] * sy : gx[h] + gy[h] * sy + gz[h] * sz);
+            if (CONTIG) {
+                const float2* __restrict__ r0 = tab + ((ALLFLAT ? gx[h] + gy[h] * sy : gx[h] + gy[h] * sy + gz[h] * sz) & mask);
                 const float2* __restrict__ r1 = r0 + sy;
                 v[i][0] = __ldg(r0); v[i][1] = __ldg(r0 + 1); v[i][2] = __ldg(r1); v[i][3] = __ldg(r1 + 1);
                 if (!ALLFLAT) {
@@ -260,11 +262,7 @@ __device__ __forceinline__ void gather3_dyn4(const GridDesc& g, int l0, float x,
                 continue;
             }
             uint32_t idx[8];
-            if (ALLFLAT) {
-                const uint32_t b = gx[h] + gy[h] * sy;
-                idx[0] = b; idx[1] = b + 1; idx[2] = b + sy; idx[3] = b + sy + 1;
-                idx[4] = idx[5] = idx[6] = idx[7] = 0;
-            } else if (hashed) {
+            if (hashed) {
                 const uint32_t y0 = gy[h] * HASH_P1, y1 = y0 + HASH_P1, z0 = gz[h] * HASH_P2, z1 = z0 + HASH_P2;
                 const uint32_t x0 = gx[h], x1 = gx[h] + 1;
                 idx[0] = x0 ^ y0 ^ z0; idx[1] = x1 ^ y0 ^ z0; idx[2] = x0 ^ y1 ^ z0; idx[3] = x1 ^ y1 ^ z0;
@@ -300,26 +298,22 @@ __device__ __forceinline__ void gather3_dyn4(const GridDesc& g, int l0, float x,
     }
 }
 
-// 1 when the n levels from l0 are all GridLevels::nowrap (uniform: level constants)
-__device__ __forceinline__ bool levels_nowrap(const GridLevels& lv, int l0, int n) {
-    bool nw = true;
+// 1 when none of the n levels from l0 is hashed (uniform: level constants)
+__device__ __forceinline__ bool levels_unhashed(const GridLevels& lv, int l0, int n) {
+    bool c = true;
     #pragma unroll
-    for (int q = 0; q < n; q++) nw = nw && lv.nowrap[l0 + q] != 0;
-    return nw;
+    for (int q = 0; q < n; q++) c = c && lv.hashed[l0 + q] == 0;
+    return c;
 }
-// unit u (levels 4u..4u+3) of the 3-D grid, with the batch's uniform ALLFLAT / NOWRAP properties
-__device__ __forceinline__ void gather3_unit(const GridDesc& g, uint32_t u, bool flat, bool nowrap, float x, float y, float z, float2 (&out)[4]) {
-    if (flat) {
-        if (nowrap) gather3_dyn4<true, true>(g, 4 * u, x, y, z, out);
-        else gather3_dyn4<true, false>(g, 4 * u, x, y, z, out);
-    } else {
-        if (nowrap) gather3_dyn4<false, true>(g, 4 * u, x, y, z, out);
-        else gather3_dyn4<false, false>(g, 4 * u, x, y, z, out);
-    }
+// unit u (levels 4u..4u+3) of the 3-D grid, with the batch's uniform ALLFLAT / CONTIG properties (ALLFLAT implies CONTIG)
+__device__ __forceinline__ void gather3_unit(const GridDesc& g, uint32_t u, bool flat, bool contig, float x, float y, float z, float2 (&out)[4]) {
+    if (flat) gather3_dyn4<true, true>(g, 4 * u, x, y, z, out);
+    else if (contig) gather3_dyn4<false, true>(g, 4 * u, x, y, z, out);
+    else gather3_dyn4<false, false>(g, 4 * u, x, y, z, out);
 }
 
-// 2-D ambient grid, 8 consecutive levels from l0 (32 gathers in flight); level pairs, channel pairs and NOWRAP as in gather3_dyn4
-template <bool NOWRAP>
+// 2-D ambient grid, 8 consecutive levels from l0 (32 gathers in flight); level pairs, channel pairs and CONTIG as in gather3_dyn4
+template <bool CONTIG>
 __device__ __forceinline__ void gather2_dyn8(const GridDesc& g, int l0, float x, float y, float2 (&out)[8]) {
     const bool oob = x < 0 || x > 1 || y < 0 || y > 1;            // tanh output mapped to [0,1]: cannot happen, kept for safety
     if (oob) { x = 0.5f; y = 0.5f; }
@@ -338,8 +332,8 @@ __device__ __forceinline__ void gather2_dyn8(const GridDesc& g, int l0, float x,
         for (int h = 0; h < 2; h++) {
             const float2* __restrict__ tab = g.lbase[l + h];
             const uint32_t mask = g.lv.mask[l + h], sy = g.lv.sy[l + h];
-            if (NOWRAP) {
-                const float2* __restrict__ r0 = tab + (gx[h] + gy[h] * sy), * __restrict__ r1 = r0 + sy;
+            if (CONTIG) {
+                const float2* __restrict__ r0 = tab + ((gx[h] + gy[h] * sy) & mask), * __restrict__ r1 = r0 + sy;
                 v[2 * k + h][0] = __ldg(r0); v[2 * k + h][1] = __ldg(r0 + 1); v[2 * k + h][2] = __ldg(r1); v[2 * k + h][3] = __ldg(r1 + 1);
                 continue;
             }
@@ -395,14 +389,14 @@ __global__ void __launch_bounds__(SPA_THREADS, 1) k_tc_amb(const SpArgs a) {
         asm volatile("setmaxnreg.inc.sync.aligned.u32 112;");
 #endif
         const uint32_t half = tid >> 7, row = tid & 127;     // half = producer warpgroup 0 .. SPA_PROD_WG-1
-        uint32_t flat_units = 0, nowrap_units = 0;     // bit u: levels 4u..4u+3 all drop z and are not hashed / are all nowrap
+        uint32_t flat_units = 0, contig_units = 0;     // bit u: levels 4u..4u+3 all drop z and are not hashed / are not hashed
         #pragma unroll
         for (int u = 0; u < 4; u++) {
             bool flat = true;
             #pragma unroll
             for (int q = 0; q < 4; q++) flat = flat && a.grid.lv.sz[4 * u + q] == 0 && a.grid.lv.hashed[4 * u + q] == 0;
             flat_units |= (flat ? 1u : 0u) << u;
-            nowrap_units |= (levels_nowrap(a.grid.lv, 4 * u, 4) ? 1u : 0u) << u;
+            contig_units |= (levels_unhashed(a.grid.lv, 4 * u, 4) ? 1u : 0u) << u;
         }
         // This warpgroup's units (4 levels each) of a row.  Two warpgroups: u = wg and wg + 2 (one 8-corner coarse unit + one z-dropped fine unit
         // each).  Three: the cheapest pair of units (cost 2 per 8-corner unit, 1 per z-dropped one) shares a warpgroup, the other two units get one each.
@@ -462,7 +456,7 @@ __global__ void __launch_bounds__(SPA_THREADS, 1) k_tc_amb(const SpArgs a) {
             for (uint32_t b = 0; b < my_nu; b++) {
                 const uint32_t u = b == 0 ? my_u0 : my_u1;
                 float2 f[4];
-                gather3_unit(a.grid, u, (flat_units >> u) & 1, (nowrap_units >> u) & 1, ux, uy, uz, f);
+                gather3_unit(a.grid, u, (flat_units >> u) & 1, (contig_units >> u) & 1, ux, uy, uz, f);
                 if (oob) { f[0] = f[1] = f[2] = f[3] = make_float2(0.f, 0.f); }
                 uint4 hi, lo;
                 pack_hilo_h2(f[0], hi.x, lo.x); pack_hilo_h2(f[1], hi.y, lo.y); pack_hilo_h2(f[2], hi.z, lo.z); pack_hilo_h2(f[3], hi.w, lo.w);
@@ -627,7 +621,7 @@ __global__ void __launch_bounds__(SP_THREADS, 1) k_tc_sigcol(const SpArgs a) {
     if (warp < 8) {
         // ------------------------------------------------ producers ------------------------------------------------
         const uint32_t half = tid >> 7, row = tid & 127;
-        const bool nowrap_half = levels_nowrap(a.grid.lv, 8 * half, 8);
+        const bool contig_half = levels_unhashed(a.grid.lv, 8 * half, 8);
         // Per-row inputs of a tile (32 B of position features, the ambient coordinate, the ray's view direction) are staged ONE TILE AHEAD with
         // cp.async -- the features and the direction straight into the NEXT ring slot, which is therefore acquired one tile early -- and the ray
         // id TWO tiles ahead, so that the dependent pos4.w -> rays_d chain never sits on a producer's critical path.  (As register prefetches the
@@ -684,7 +678,7 @@ __global__ void __launch_bounds__(SP_THREADS, 1) k_tc_sigcol(const SpArgs a) {
             }
             const float vx = (ap.x + 1.0f) * 0.5f, vy = (ap.y + 1.0f) * 0.5f;
             float2 f[8];
-            if (nowrap_half) gather2_dyn8<true>(a.grid, 8 * half, vx, vy, f);
+            if (contig_half) gather2_dyn8<true>(a.grid, 8 * half, vx, vy, f);
             else gather2_dyn8<false>(a.grid, 8 * half, vx, vy, f);
             #pragma unroll
             for (int u = 0; u < 2; u++)
@@ -864,7 +858,7 @@ __global__ void __launch_bounds__(256) k_gather_probe(GridDesc pos, GridDesc amb
         #pragma unroll
         for (int q = 0; q < 4; q++) flat = flat && pos.lv.sz[4 * u + q] == 0 && pos.lv.hashed[4 * u + q] == 0;
         float2 f[4];
-        gather3_unit(pos, u, flat, levels_nowrap(pos.lv, 4 * u, 4), ux, uy, uz, f);
+        gather3_unit(pos, u, flat, levels_unhashed(pos.lv, 4 * u, 4), ux, uy, uz, f);
         #pragma unroll
         for (int q = 0; q < 4; q++) { acc.x += f[q].x; acc.y += f[q].y; }
     }
@@ -873,7 +867,7 @@ __global__ void __launch_bounds__(256) k_gather_probe(GridDesc pos, GridDesc amb
     #pragma unroll 1
     for (int h = 0; h < 2; h++) {
         float2 f[8];
-        if (levels_nowrap(amb.lv, 8 * h, 8)) gather2_dyn8<true>(amb, 8 * h, vx, vy, f);
+        if (levels_unhashed(amb.lv, 8 * h, 8)) gather2_dyn8<true>(amb, 8 * h, vx, vy, f);
         else gather2_dyn8<false>(amb, 8 * h, vx, vy, f);
         #pragma unroll
         for (int q = 0; q < 8; q++) { acc.x += f[q].x; acc.y += f[q].y; }

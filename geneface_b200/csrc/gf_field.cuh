@@ -21,12 +21,15 @@ struct GridLevels {
     uint32_t sz[16];       // stride of z (0 when dropped; unused for 2-D grids)
     uint32_t mask[16];     // index & mask  ==  index % hsize
     uint32_t hashed[16];   // 1: fast_hash index (gridtype 0 on a clipped level)
-    uint32_t nowrap[16];   // 1: dense level whose largest corner index stays below hsize: the mask never changes an index
+    // Wrapping levels (not hashed, and the largest corner index reaches hsize, so `& mask` changes it) are read from a padded image:
+    // E[k] = T[k % hsize] for k < hsize + pad, pad = 1 + sy + sz (the largest corner offset).  Then E[(b & mask) + d] == T[(b + d) & mask]
+    // for every corner offset d, so the corners of a cell are rows of adjacent entries.  pad = 0 on every other level.
+    uint32_t pad[16];
+    uint32_t img_offset[16];   // first entry of the level in the padded image (levels of hsize + pad entries, level-major)
 };
 
 struct GridDesc {
-    const float2* table;   // [sum hsize] entries of 2 floats
-    const float2* lbase[16];   // table + offset[l]: one 64-bit base per level (address = IMAD.WIDE(idx, 8, base))
+    const float2* lbase[16];   // first entry of level l (padded image: img_offset[l]; table read in place: offset[l]); address = IMAD.WIDE(idx, 8, base)
     GridLevels lv;
     uint32_t gridtype;     // 0 hash, 1 tiled
     uint32_t interp;       // 0 linear, 1 smoothstep

@@ -123,6 +123,7 @@ struct GfModel {
     float* w;               // packed fp32 blob (device)
     size_t w_floats;
     float w_amb2_host[256]; // fp32 ambient output layer [2][128] (host copy, passed by value to k_tc_amb)
+    float2* grid_img;       // padded images of the position and ambient grid tables (device, one allocation; GridLevels::pad)
     void* tc2_blob;         // fp16 weight images of the two tcgen05 kernels (device), built in gf_model_create; null outside the envelope
     float* tc_dbg;          // diagnostics buffer for the tcgen05 kernel (gf_tc_debug) or null
     int num_sms;

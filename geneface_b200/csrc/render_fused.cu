@@ -37,34 +37,55 @@ namespace gf {
 // ======================================================================================
 // model setup kernels
 // ======================================================================================
+// one warp: lane l < 16 computes level l, all 32 lanes take part in the scan of the padded image's level sizes
 __global__ void k_level_geometry(const int* __restrict__ offsets, float S, uint32_t H, uint32_t D, uint32_t gridtype, GridLevels* out,
                                  int* __restrict__ bad) {
     const int l = threadIdx.x;
-    if (l >= 16) return;
-    // gridencoder.cu:137-139 (device exp2f on purpose: bit-identical scale to the reference kernel)
-    const float scale = __fmaf_rn(exp2f(__fmul_rn((float)l, S)), (float)H, -1.0f);
-    const uint32_t res = (uint32_t)ceilf(scale) + 1;
-    const uint32_t hs = (uint32_t)(offsets[l + 1] - offsets[l]);
-    out->scale[l] = scale;
-    out->res[l] = res;
-    out->hsize[l] = hs;
-    out->offset[l] = (uint32_t)offsets[l];
-    // replay of the stride loop of get_grid_index (gridencoder.cu:68-75, align_corners = false), uint32 wrap-around included
-    const uint32_t R = res + 1;
-    uint32_t stride = 1, sy = 0, sz = 0;
-    stride *= R;                                              // d = 0 is always taken (1 <= hashmap_size)
-    if (stride <= hs) { sy = stride; stride *= R; }
-    if (D == 3 && stride <= hs) { sz = stride; stride *= R; }
-    out->sy[l] = sy;
-    out->sz[l] = sz;
-    out->hashed[l] = (gridtype == 0 && stride > hs) ? 1u : 0u;
-    const bool pow2 = hs && (hs & (hs - 1)) == 0;
-    out->mask[l] = pow2 ? hs - 1 : 0xFFFFFFFFu;
-    // `index % hsize` is only replaced by the mask when it is provably the same: power-of-two level, or a dense level
-    // whose largest reachable index (pos_grid <= res per axis) stays below hsize.
-    const unsigned long long maxidx = (unsigned long long)res * (1ull + sy + sz);
-    out->nowrap[l] = (!out->hashed[l] && maxidx < hs) ? 1u : 0u;
-    if (!pow2 && !out->nowrap[l]) *bad = 1;
+    uint32_t entries = 0;          // entries of level l in the padded image
+    if (l < 16) {
+        // gridencoder.cu:137-139 (device exp2f on purpose: bit-identical scale to the reference kernel)
+        const float scale = __fmaf_rn(exp2f(__fmul_rn((float)l, S)), (float)H, -1.0f);
+        const uint32_t res = (uint32_t)ceilf(scale) + 1;
+        const uint32_t hs = (uint32_t)(offsets[l + 1] - offsets[l]);
+        out->scale[l] = scale;
+        out->res[l] = res;
+        out->hsize[l] = hs;
+        out->offset[l] = (uint32_t)offsets[l];
+        // replay of the stride loop of get_grid_index (gridencoder.cu:68-75, align_corners = false), uint32 wrap-around included
+        const uint32_t R = res + 1;
+        uint32_t stride = 1, sy = 0, sz = 0;
+        stride *= R;                                              // d = 0 is always taken (1 <= hashmap_size)
+        if (stride <= hs) { sy = stride; stride *= R; }
+        if (D == 3 && stride <= hs) { sz = stride; stride *= R; }
+        out->sy[l] = sy;
+        out->sz[l] = sz;
+        const bool hashed = gridtype == 0 && stride > hs;
+        out->hashed[l] = hashed ? 1u : 0u;
+        const bool pow2 = hs && (hs & (hs - 1)) == 0;
+        out->mask[l] = pow2 ? hs - 1 : 0xFFFFFFFFu;
+        // `index % hsize` is only replaced by the mask when it is provably the same: power-of-two level, or a dense level
+        // whose largest reachable index (pos_grid <= res per axis) stays below hsize.
+        const unsigned long long maxidx = (unsigned long long)res * (1ull + sy + sz);
+        const bool nowrap = !hashed && maxidx < hs;
+        if (!pow2 && !nowrap) *bad = 1;
+        const uint32_t pad = (hashed || nowrap) ? 0u : 1u + sy + sz;
+        out->pad[l] = pad;
+        entries = hs + pad;
+    }
+    uint32_t incl = entries;
+    #pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const uint32_t v = __shfl_up_sync(0xFFFFFFFFu, incl, o);
+        if (l >= o) incl += v;
+    }
+    if (l < 16) out->img_offset[l] = incl - entries;
+}
+
+// padded image of a grid table (GridLevels::pad): dst[img_offset[l] + k] = src[offset[l] + k % hsize[l]], k < hsize[l] + pad[l]
+__global__ void k_grid_image(const float2* __restrict__ src, const GridLevels lv, float2* __restrict__ dst) {
+    const uint32_t l = blockIdx.y, hs = lv.hsize[l], n = hs + lv.pad[l];
+    for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x)
+        dst[lv.img_offset[l] + k] = src[lv.offset[l] + k % hs];
 }
 
 // dst[k][n] = src[n][k0 + k]   (src row-major [N][ldsrc]); dst row stride ldd
@@ -852,16 +873,31 @@ GF_API int gf_model_create(const GfModelDesc* d, GfModel** out, gf_stream_t stre
         delete m;
         return GF_ERR_CUDA;
     }
-    md.pos.table = reinterpret_cast<const float2*>(d->pos_embeddings); md.pos.lv = lv_host[0]; md.pos.gridtype = d->gridtype; md.pos.interp = d->interp;
-    md.amb.table = reinterpret_cast<const float2*>(d->amb_embeddings); md.amb.lv = lv_host[1]; md.amb.gridtype = d->gridtype; md.amb.interp = d->interp;
-    md.torso.table = reinterpret_cast<const float2*>(d->torso_embeddings); md.torso.lv = lv_host[2]; md.torso.gridtype = 1; md.torso.interp = 0;   // radnerf_torso.py:36 ('tiledgrid', linear)
+    md.pos.lv = lv_host[0]; md.pos.gridtype = d->gridtype; md.pos.interp = d->interp;
+    md.amb.lv = lv_host[1]; md.amb.gridtype = d->gridtype; md.amb.interp = d->interp;
+    md.torso.lv = lv_host[2]; md.torso.gridtype = 1; md.torso.interp = 0;   // radnerf_torso.py:36 ('tiledgrid', linear)
+    // Padded images of the position and ambient tables (GridLevels::pad): the field kernels' producers address every non-hashed level's
+    // corners as rows of adjacent entries.  Copied here, like the weights; the torso table is read in place.
+    auto img_entries = [](const GridLevels& lv) { return (size_t)lv.img_offset[15] + lv.hsize[15] + lv.pad[15]; };
+    const size_t pos_n = img_entries(lv_host[0]), amb_n = img_entries(lv_host[1]);
+    if (cudaMalloc(&m->grid_img, (pos_n + amb_n) * sizeof(float2)) != cudaSuccess) {
+        cudaGetLastError();
+        set_error("model_create: cudaMalloc of the grid images failed");
+        gf_model_destroy(m);
+        return GF_ERR_CUDA;
+    }
+    const dim3 img_grid(256, 16);        // grid-stride over each level
+    k_grid_image<<<img_grid, 256, 0, st>>>(reinterpret_cast<const float2*>(d->pos_embeddings), lv_host[0], m->grid_img);
+    k_grid_image<<<img_grid, 256, 0, st>>>(reinterpret_cast<const float2*>(d->amb_embeddings), lv_host[1], m->grid_img + pos_n);
+    if (int rc = check_launch("model_create: grid images")) { gf_model_destroy(m); return rc; }
+    const float2* torso_tab = reinterpret_cast<const float2*>(d->torso_embeddings);
     for (int l = 0; l < 16; l++) {
-        md.pos.lbase[l] = md.pos.table + lv_host[0].offset[l];
-        md.amb.lbase[l] = md.amb.table + lv_host[1].offset[l];
-        md.torso.lbase[l] = md.torso.table ? md.torso.table + lv_host[2].offset[l] : nullptr;
+        md.pos.lbase[l] = m->grid_img + lv_host[0].img_offset[l];
+        md.amb.lbase[l] = m->grid_img + pos_n + lv_host[1].img_offset[l];
+        md.torso.lbase[l] = torso_tab ? torso_tab + lv_host[2].offset[l] : nullptr;
     }
     // fp16 weight images of the tcgen05 pipeline (field_tc_split.cu): packed here, once -- the frame path never allocates or synchronises
-    if (int prc = field_tc_pack(m, st)) { cudaFree(w); delete m; return prc; }
+    if (int prc = field_tc_pack(m, st)) { gf_model_destroy(m); return prc; }
     cudaFuncSetAttribute(k_field_fp32, cudaFuncAttributeMaxDynamicSharedMemorySize, FP32_SMEM_FLOATS * (int)sizeof(float));
     cudaFuncSetAttribute(k_torso_field, cudaFuncAttributeMaxDynamicSharedMemorySize, TORSO_SMEM_FLOATS * (int)sizeof(float));
     int dev = 0;
@@ -875,6 +911,7 @@ GF_API int gf_model_create(const GfModelDesc* d, GfModel** out, gf_stream_t stre
 GF_API void gf_model_destroy(GfModel* m) {
     if (!m) return;
     if (m->w) cudaFree(m->w);
+    if (m->grid_img) cudaFree(m->grid_img);
     if (m->tc2_blob) cudaFree(m->tc2_blob);
     for (int i = 0; i < GF_MAX_PROFILE_EVENTS; i++)
         if (m->ev[i]) cudaEventDestroy(m->ev[i]);

@@ -210,7 +210,8 @@ class NeRFRenderer(nn.Module):
         """Drop the packed GfModel (and every captured frame graph): the next fused call re-packs from the live tensors.
         Called automatically by load_state_dict / train() / eval() / _apply (.to, .cuda, .half) and by the grid-maintenance
         routines; call it yourself after in-place edits that bypass autograd's version counter (`p.data.copy_`, EMA weight
-        surgery, optimizers writing through .data)."""
+        surgery, optimizers writing through .data).  That includes edits of the position and ambient grid tables: the packed model
+        reads padded copies of them, made when it is built."""
         self._gf_key = None
         self._gf_epoch = getattr(self, '_gf_epoch', 0) + 1
 

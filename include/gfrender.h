@@ -223,8 +223,9 @@ GF_API int gf_tl_wgrad(const void* p, uint32_t p_chunks, uint32_t p_c0, const vo
 typedef struct GfModel GfModel;
 
 /* Raw device pointers to the reference's state_dict tensors (SURVEY.md section 8a).  Not retained
- * after gf_model_create returns (weights are repacked into the model's own buffers);
- * the three grid tables and the bitfields ARE referenced in place (no copy). */
+ * after gf_model_create returns (weights are repacked into the model's own buffers, and the
+ * position and ambient grid tables are copied into padded model-owned images);
+ * the torso grid table and the bitfields ARE referenced in place (no copy). */
 typedef struct GfModelDesc {
     /* geometry / hyper-parameters */
     float bound;                 /* hparams['bound']                       renderer.py:66 */
